@@ -335,6 +335,40 @@ def _emit(line):
     os.write(_RESULT_FD if _RESULT_FD is not None else 1, data)
 
 
+DUMP_BYTES = 64 * 10 ** 6      # --dump-outputs: every .npy file together, headers included, stays under this
+
+
+def snapshot_outputs(arrays, budget=DUMP_BYTES - 64 * 1024):
+    """Host copies of the arrays one timed step returned, for --dump-outputs: float64 stays float64 and so do integer
+    tensors (exact below 2**53), every other dtype becomes float32.  The arrays are taken smallest first, each whole if it
+    fits its even share of what is left of the budget; a larger one is replaced by a fixed sample of k of its flattened
+    elements, `np.random.default_rng(0).choice(numel, k, replace=False)` in ascending order, so the same shapes always
+    yield the same positions.  Taken right after the timed loop: graph replays write into the same output buffers, so
+    later work would overwrite them."""
+    import numpy as np
+    import torch
+    ts = {name: torch.as_tensor(t).detach() for name, t in arrays.items()}
+    out, left = {}, budget
+    for i, name in enumerate(sorted(ts, key=lambda n: ts[n].numel())):
+        t = ts[name]
+        dt = torch.float32 if t.is_floating_point() and t.dtype != torch.float64 else torch.float64
+        k = left // (len(ts) - i) // dt.itemsize
+        if t.numel() > k:
+            idx = np.sort(np.random.default_rng(0).choice(t.numel(), size=k, replace=False))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        out[name] = t.to(dt).cpu().numpy()
+        left -= out[name].nbytes
+    return {name: out[name] for name in arrays}
+
+
+def write_outputs(directory, arrays):
+    """--dump-outputs: DIR/<name>.npy for every array snapshot_outputs() kept."""
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
+
+
 def run_train_step(args, rank, local_rank, world):
     """`--workload train-step` (BASELINE config 4, SURVEY section 8 a22 + e): one v1 consistency-distillation step per rank on one
     16x320x512 sample (latents 1x4x16x40x64, 77x1024 prompt embeddings): add_noise, the LoRA-injected student forward
@@ -404,6 +438,8 @@ def run_train_step(args, rank, local_rank, world):
     e1.record()
     t2v_dist.barrier(device)
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:     # what train_step returned for the last timed step
+        write_outputs(args.dump_outputs, snapshot_outputs(out))
     ms = e0.elapsed_time(e1)
     launches = ops.LAUNCHES - n0
     finite = bool(torch.isfinite(out["loss"]).all()) and bool(torch.isfinite(student.arena.params).all())
@@ -521,6 +557,8 @@ def run_v2_step(args, rank, local_rank, world):
     e1.record()
     t2v_dist.barrier(device)
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:     # what train_step_v2 returned for the last timed step
+        write_outputs(args.dump_outputs, snapshot_outputs(out))
     ms = t2v_dist.max_over_ranks([e0.elapsed_time(e1)], device)[0]
     finite = bool(torch.isfinite(out["loss"]).all()) and bool(torch.isfinite(student.arena.params).all())
     launches = (ops.LAUNCHES - n0) + (launches_per_step * args.steps if use_graph else 0)
@@ -636,6 +674,8 @@ def run_lora_step(args, rank, local_rank, world):
     e1.record()
     t2v_dist.barrier(device)
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:     # the step returns nothing: its results are the updated LoRA parameters and their gradients
+        write_outputs(args.dump_outputs, snapshot_outputs(dict(params=arena.params, grads=arena.grads)))
     ms = e0.elapsed_time(e1)
     launches = ops.LAUNCHES - n0
     # the exchange alone (same buffer, no overlap), for the all-reduce share
@@ -678,7 +718,14 @@ def main():
     ap.add_argument("--motion-cond", action="store_true", help="VC2 pipeline with the v2 motion conditioning (BASELINE configs[2])")
     ap.add_argument("--workload", default="pipeline", choices=["pipeline", "ms-pipeline", "lora-step", "train-step", "v2-step"],
                     help="pipeline = the headline metric; lora-step = the data-parallel LoRA training exchange (supplementary)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned as DIR/<name>.npy (float32 / float64, at most "
+                         "64 MB in all: larger outputs as a fixed seeded sample); the inputs depend only on the arguments")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs: the reference arm only times a bounded sample of the workload and returns no outputs")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -736,6 +783,8 @@ def main():
     e1.record()
     barrier()
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:     # the decoded videos of the last timed call
+        write_outputs(args.dump_outputs, snapshot_outputs(dict(video=vid)))
     ms = e0.elapsed_time(e1)
     finite = bool(torch.isfinite(vid.float()).all())
 

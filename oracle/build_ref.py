@@ -32,6 +32,8 @@ def build_ref(src: str = SRC, dst: str = DST) -> str | None:
                 os.makedirs(os.path.join(dst, rel), exist_ok=True)
                 shutil.copyfile(os.path.join(root, f), os.path.join(dst, rel, f))
                 n += 1
+    if n == 0:          # present but empty or unreadable: no snapshot
+        return None
     with open(os.path.join(dst, "SNAPSHOT.txt"), "w") as fh:
         fh.write(f"verbatim copy of {n} .py files of {src} ({', '.join(PACKAGES)}) made by oracle/build_ref.py; not committed\n")
     return dst

@@ -705,6 +705,41 @@ def gen_scheduler():
     print("  scheduler: alphas_cumprod[0], [999] =", float(s.alphas_cumprod[0]), float(s.alphas_cumprod[999]))
 
 
+def gen_scheduler_bf16_cuda():
+    """The reference scheduler's bf16 steps EXECUTED ON A CUDA DEVICE (run where one is): torch's CUDA kernels keep the 0-dim
+    fp32 coefficients in fp32, so these differ from the CPU `steps_bf16` of scheduler.pt by a few ulps and are what the fused
+    step kernel reproduces bit for bit.  Needs a copy of the reference (oracle/_ref/ or the source tree) and a GPU."""
+    from oracle import ref_loader
+    assert ref_loader.enable() is not None, "no copy of the reference"
+    from scheduler.t2v_turbo_scheduler import T2VTurboScheduler
+    assert torch.cuda.is_available(), "the CUDA arithmetic of the reference needs a GPU"
+    g = torch.load(os.path.join(GOLD, "scheduler.pt"))
+    s = T2VTurboScheduler(linear_start=0.00085, linear_end=0.012)
+    s.set_timesteps(4, 50)
+    xb, eb = g["x"].bfloat16().cuda(), g["eps"].bfloat16().cuda()
+    steps = []
+    for st in g["steps_bf16"]:
+        prev, den = s.step(eb, st["i"], s.timesteps[st["i"]], xb, generator=torch.Generator().manual_seed(100 + st["i"]), return_dict=False)
+        steps.append({"i": st["i"], "t": int(s.timesteps[st["i"]]), "prev": prev.cpu(), "den": den.cpu()})
+    torch.save({"device": torch.cuda.get_device_name(0), "torch": str(torch.__version__), "steps": steps},
+               os.path.join(GOLD, "scheduler_bf16_cuda.pt"))
+    print("  scheduler bf16 on", torch.cuda.get_device_name(0))
+
+
+def gen_lora_traversal():
+    """(name, weight shape) of every Linear / Conv2d / Conv3d of the reference UNetModel on the `mid` config, in
+    named_modules() order: the order utils/lora.py injects LoRA layers in."""
+    import json
+    from lvdm.modules.networks.openaimodel3d import UNetModel
+    cfg = UNET_CONFIGS["mid"]["cfg"]
+    m = UNetModel(**cfg)
+    rows = [[n, list(mod.weight.shape)] for n, mod in m.named_modules()
+            if mod.__class__ in (torch.nn.Linear, torch.nn.Conv2d, torch.nn.Conv3d)]
+    with open(os.path.join(GOLD, "lora_traversal_mid.json"), "w") as f:
+        f.write('{"config": "mid", "layers": [\n' + ",\n".join(json.dumps(r) for r in rows) + "\n]}\n")
+    print(f"  lora traversal: {len(rows)} layers")
+
+
 def _ref_pipeline(unet_name):
     """The unmodified reference pipeline around a small UNet / VAE (the attributes it touches: pipeline:27-29,144,216)."""
     from pipeline.t2v_turbo_vc2_pipeline import T2VTurboVC2Pipeline
@@ -797,11 +832,15 @@ if __name__ == "__main__":
     a = ap.parse_args()
     os.makedirs(GOLD, exist_ok=True)
     torch.set_num_threads(os.cpu_count())
-    todo = a.only.split(",") if a.only else ["scheduler", "unet_small", "unet_mid", "vae_small", "vae_enc_small", "lora_small", "pipeline", "unet_small_motion", "pipeline_v2", "lora_layers", "unet_probs", "student_grads", "distill_step", "distill_tables", "v2_step", "full_grads", "motion_score", "preprocess_sample", "student_grads_mid"] + (["unet_full", "vae_full", "vae_enc_full", "unet_full_t", "unet_full_b2"] if a.full else [])
+    todo = a.only.split(",") if a.only else ["scheduler", "unet_small", "unet_mid", "vae_small", "vae_enc_small", "lora_small", "pipeline", "unet_small_motion", "pipeline_v2", "lora_layers", "unet_probs", "student_grads", "distill_step", "distill_tables", "v2_step", "full_grads", "motion_score", "preprocess_sample", "student_grads_mid", "lora_traversal"] + (["unet_full", "vae_full", "vae_enc_full", "unet_full_t", "unet_full_b2"] if a.full else [])
     for item in todo:
         print("generating", item)
         if item == "scheduler":
             gen_scheduler()
+        elif item == "scheduler_bf16_cuda":    # not in the default list: needs a GPU
+            gen_scheduler_bf16_cuda()
+        elif item == "lora_traversal":
+            gen_lora_traversal()
         elif item.startswith("unet_") and item != "unet_probs":
             gen_unet(item[5:])
         elif item == "lora_layers":

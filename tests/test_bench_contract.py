@@ -51,3 +51,24 @@ def test_two_gpu_line_is_weak_scaling_aggregate():
     one, two = _load("r02_bench_default.json"), _load("r02_bench_2gpu.json")
     assert two["n_gpus"] == 2 and two["scaling"] == "weak"
     assert 1.8 < two["value"] / one["value"] < 2.2
+
+
+def test_dump_outputs_sample_is_fixed_and_within_budget(tmp_path):
+    """bench.py --dump-outputs: float32 / float64 files, small arrays whole, a large one as the same seeded sample every time,
+    everything within the byte budget."""
+    import numpy as np
+    import torch
+
+    import bench
+    arrays = dict(video=torch.arange(3000.0).reshape(3, 1000), loss=torch.tensor([0.5], dtype=torch.bfloat16),
+                  index=torch.tensor([7, 9]), w=torch.tensor([2.5], dtype=torch.float64))
+    a, b = bench.snapshot_outputs(arrays, budget=4000), bench.snapshot_outputs(arrays, budget=4000)
+    assert list(a) == list(arrays)
+    assert {k: v.dtype for k, v in a.items()} == dict(video=np.float32, loss=np.float32, index=np.float64, w=np.float64)
+    assert a["index"].tolist() == [7, 9] and a["w"].tolist() == [2.5] and a["loss"].shape == (1,)
+    assert sum(v.nbytes for v in a.values()) <= 4000 and 0 < a["video"].size < 3000
+    assert np.array_equal(a["video"], b["video"])
+    assert np.all(np.diff(a["video"]) > 0) and np.all(a["video"] == np.round(a["video"]))   # ascending positions of the flattened array
+    bench.write_outputs(str(tmp_path / "out"), a)
+    assert sorted(os.listdir(tmp_path / "out")) == ["index.npy", "loss.npy", "video.npy", "w.npy"]
+    assert np.array_equal(np.load(tmp_path / "out" / "video.npy"), a["video"])

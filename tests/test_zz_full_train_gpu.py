@@ -182,7 +182,16 @@ def test_v2_step_vs_reference_composition(cuda_device):
     loss, loss_ref = float(out["loss"]), float(g["loss"])
     print(f"\n[v2 small] loss {loss:.6f} vs reference {loss_ref:.6f}; rel-L2 {e}")
     assert e["x_prev"] < 1e-5 and e["model_pred"] < 1.4e-2 and e["target"] < 1.3e-2, e          # observed 1.3e-6 / 6.7e-3 / 6.4e-3
-    assert abs(loss - loss_ref) < 2e-3 * loss_ref, (loss, loss_ref)                                # observed 8.9e-4
+    # The loss is the pseudo-Huber mean of OUR model_pred - target (fp64 recomputation), and it departs from the reference loss
+    # by no more than the forward departures above allow: the pseudo-Huber function is 1-Lipschitz, so |loss - loss_ref| <=
+    # mean |(p - t) - (p_ref - t_ref)|.  A fixed bound on |loss - loss_ref| is not a property of the code: the fp32 atomics make
+    # each run a different bf16 rounding pattern, and on these 2 048 elements the loss moved by 8.9e-4 and by 2.2e-3 between runs.
+    d, d_ref = (out["model_pred"] - out["target"]).double().cpu(), (g["model_pred"] - g["target"]).double()
+    c = 0.001                                                                                  # V2Step's default huber_c
+    own = float(((d * d + c * c).sqrt() - c).mean())
+    assert abs(loss - own) < 1e-5 * own, (loss, own)
+    assert abs(loss - loss_ref) <= float((d - d_ref).abs().mean()) + 1e-6, (loss, loss_ref, float((d - d_ref).abs().mean()))
+    assert abs(loss - loss_ref) < 1e-2 * loss_ref, (loss, loss_ref)
     names = s.arena.names
     gv = s.arena.grad
     assert torch.isfinite(s.arena.grads).all()
